@@ -266,6 +266,19 @@ def workload_config(name, params, gpus):
 
 
 # ====================================================================== GPU arm
+def dump_outputs(directory, name, sample, rank, world):
+    """``--dump-outputs``: the sampled results of the last timed step as ``<name>.npy``
+    (``<name>_rank<r>.npy`` on more than one GPU), float64 (result, pixel, re / im).  The
+    pixels are the same seeded sample of every result, and the inputs of every step come from
+    fixed seeds, so two builds can be compared output for output.  The forward sample is
+    gathered on the device inside the last timed step (one small gather per subgrid)."""
+    os.makedirs(directory, exist_ok=True)
+    fname = name if world == 1 else f"{name}_rank{rank}"
+    arr = sample.array()
+    numpy.save(os.path.join(directory, fname + ".npy"), arr)
+    note(f"wrote {fname}.npy {arr.shape} to {directory}")
+
+
 def main_gpu(args):
     # Everything but the final JSON line goes to stderr -- also what libraries print on the C
     # level (NCCL writes its version banner to stdout when the first communicator is created).
@@ -302,10 +315,20 @@ def _main_gpu_backward(args, dev, rank, world):
         sampler.start()
     times = []
     for i in range(args.steps):
-        times.append(runner.step(timed=True))
+        if args.dump_outputs and i == args.steps - 1:
+            ms, tasks = runner.step(timed=True, keep=True)
+            sample = bs.OutputSample(tasks[0].tensor.shape, len(tasks), dev)
+            for j, task in enumerate(tasks):
+                sample(j, None, task.tensor)
+            del tasks
+            times.append(ms)
+        else:
+            times.append(runner.step(timed=True))
         note(f"timed step {i + 1}/{args.steps}: {times[-1]:.1f} ms "
              f"(subgrids {runner.last_parts[0]:.1f} + finish {runner.last_parts[1]:.1f})")
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "facets", sample, rank, world)
     ms = float(numpy.mean(times))
     parity = None if args.no_selfcheck else runner.selfcheck()
     extra = runner.kernel_rooflines(hbm_gbs) if not args.no_roofline else None
@@ -374,10 +397,16 @@ def _main_gpu(args):
     if rank == 0:
         sampler.start()
     times = []
+    sample = None
     for i in range(args.steps):
-        times.append(runner.step(timed=True))
+        if args.dump_outputs and i == args.steps - 1:
+            owned = [j for j in range(len(runner.sg_cfgs)) if j % world == rank]
+            sample = bs.OutputSample((runner.xA, runner.xA), len(owned), dev)
+        times.append(runner.step(timed=True, consumer=sample))
         note(f"timed step {i + 1}/{args.steps}: {times[-1]:.1f} ms")
     clocks = sampler.stop() if rank == 0 else None
+    if sample is not None:
+        dump_outputs(args.dump_outputs, "subgrids", sample, rank, world)
     ms = float(numpy.mean(times))
     contributions = runner.contributions_per_step
     value = contributions / (ms * 1e-3)
@@ -450,10 +479,17 @@ def main():
     ap.add_argument("--selfcheck", action="store_true", help="(default) kept for symmetry")
     ap.add_argument("--e2e-steps", type=int, default=1)
     ap.add_argument("--cpu-cores", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed, seeded sample of every result of the last timed step "
+                         "to DIR/<name>.npy (float64, at most 64 MB)")
     ap.add_argument("--exchange", default="auto", choices=["auto", "copy", "p2p", "nccl"],
                     help="multi-GPU strip exchange: copy engines on peer memory (auto), TMA "
                          "stores into peer memory, or NCCL all_to_all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs the GPU implementation")
     if args.impl == "reference":
         main_reference(args)
     else:

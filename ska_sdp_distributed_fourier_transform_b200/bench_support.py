@@ -27,6 +27,28 @@ from .fourier_algorithm import make_subgrid_from_sources
 MIB = float(1 << 20)
 
 
+class OutputSample:
+    """The same seeded sample of pixels from each of ``count`` results of one ``shape``,
+    gathered on the device as the results appear; at most ``max_bytes`` in all."""
+
+    def __init__(self, shape, count, device, max_pixels=2048, max_bytes=64 * 2**20):
+        size = int(numpy.prod(shape))
+        n = max(1, min(max_pixels, size, max_bytes // (16 * max(1, count))))
+        idx = numpy.sort(numpy.random.default_rng(20261017).choice(size, n, replace=False))
+        self.idx = torch.from_numpy(idx).to(device)
+        self.rows = {}
+        # load the gather kernel now: a first use inside a timed step would pay for it there
+        tiny = torch.zeros(1, dtype=torch.complex128, device=device)
+        tiny[torch.zeros(1, dtype=torch.int64, device=device)].cpu()
+
+    def __call__(self, i, _config, tensor):
+        self.rows[i] = torch.view_as_real(tensor.reshape(-1)[self.idx])
+
+    def array(self):
+        """float64 array (results in order, pixels, real / imaginary part)."""
+        return numpy.stack([self.rows[i].cpu().numpy() for i in sorted(self.rows)])
+
+
 class ForwardBenchRunner:
     """Synthetic full-cover forward transform of one parameter set on ``world`` GPUs."""
 
@@ -113,14 +135,15 @@ class ForwardBenchRunner:
             dist.barrier()
         torch.cuda.synchronize(self.device)
 
-    def step(self, timed=True):
-        """One complete forward transform; returns its time in ms (max over ranks)."""
+    def step(self, timed=True, consumer=None):
+        """One complete forward transform; returns its time in ms (max over ranks).
+        ``consumer(i, subgrid_config, tensor)`` sees every subgrid this rank finishes."""
         self.regenerate_facets()
         self._barrier()
         start = torch.cuda.Event(enable_timing=True)
         end = torch.cuda.Event(enable_timing=True)
         start.record()
-        self._run_forward(self.facet_views)
+        self._run_forward(self.facet_views, consumer=consumer)
         end.record()
         self._barrier()
         ms = start.elapsed_time(end)

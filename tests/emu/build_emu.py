@@ -6,6 +6,7 @@ plain g++ and -DSWIFTLY_EMU; CUDA threads run as fibres (emu_runtime.h).  Used
 only by tests marked "not gpu" to check kernel index algebra without a GPU.
 """
 
+import fcntl
 import glob
 import os
 import subprocess
@@ -39,20 +40,31 @@ def build(force=False, opt="-O1"):
         return OUT
     objdir = os.path.join(HERE, "build")
     os.makedirs(objdir, exist_ok=True)
-    procs = []
-    objs = []
-    for src in sources():
-        obj = os.path.join(objdir, os.path.basename(src) + ".o")
-        objs.append(obj)
-        cmd = ["g++", "-std=c++17", opt, "-fPIC", "-x", "c++", "-DSWIFTLY_EMU", "-I", HERE,
-               "-I", os.path.join(ROOT, "include"), "-Wno-unknown-pragmas", "-c", src, "-o", obj]
-        procs.append((cmd, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT)))
-    for cmd, p in procs:
-        out, _ = p.communicate()
-        if p.returncode != 0:
-            sys.stderr.write(out.decode())
-            raise RuntimeError("emulator build failed: " + " ".join(cmd))
-    subprocess.check_call(["g++", "-shared", "-o", OUT] + objs)
+    # Several test processes (the spawned ranks of tests/test_dist_gloo.py) may ask for the
+    # library at once: one builds while the others wait, and the library appears under its
+    # name only once it is completely linked.
+    with open(os.path.join(objdir, "build.lock"), "w") as lock:
+        fcntl.flock(lock, fcntl.LOCK_EX)
+        if not force and up_to_date():
+            return OUT
+        procs = []
+        objs = []
+        for src in sources():
+            obj = os.path.join(objdir, os.path.basename(src) + ".o")
+            objs.append(obj)
+            cmd = ["g++", "-std=c++17", opt, "-fPIC", "-x", "c++", "-DSWIFTLY_EMU", "-I", HERE,
+                   "-I", os.path.join(ROOT, "include"), "-Wno-unknown-pragmas", "-c", src, "-o",
+                   obj]
+            procs.append((cmd, subprocess.Popen(cmd, stdout=subprocess.PIPE,
+                                                stderr=subprocess.STDOUT)))
+        for cmd, p in procs:
+            out, _ = p.communicate()
+            if p.returncode != 0:
+                sys.stderr.write(out.decode())
+                raise RuntimeError("emulator build failed: " + " ".join(cmd))
+        tmp = os.path.join(objdir, os.path.basename(OUT) + ".tmp")
+        subprocess.check_call(["g++", "-shared", "-o", tmp] + objs)
+        os.replace(tmp, OUT)
     return OUT
 
 

@@ -2,19 +2,18 @@
 """
 Generate golden fixtures from the REAL reference implementation.
 
-Run in the build container only (``/root/reference`` does not exist on the GPU
-box):
+Run where a checkout of the reference (ska-sdp-exec-swiftly) exists:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference checkout>/src [fixture ...]
 
 It imports the unmodified reference package ``ska_sdp_exec_swiftly`` (numpy
-backend ``SwiftlyCore`` and the ``api_helper`` task bodies) from
-``/root/reference/src`` -- with tiny stub modules standing in for the
+backend ``SwiftlyCore`` and the ``api_helper`` task bodies) from the given
+source directory -- with tiny stub modules standing in for the
 uninstallable ``dask`` / ``distributed`` / ``ska_sdp_func`` imports, exactly as
 described in SURVEY.md Appendix A -- runs it on seeded inputs and stores inputs
-and outputs as ``tests/golden/*.npz``.  Those files pin the oracle
-(``tests/test_oracle.py``) and, on the GPU, the CUDA path
-(``tests/test_gpu_golden.py``).
+and outputs as ``tests/golden/*.npz`` (all of them, or only the named fixtures:
+``1d``, ``2d``, ``windows``, ``dropin``).  Those files pin the oracle
+(``tests/test_oracle.py``) and the kernels (``tests/test_emu_reference_dropin.py``).
 """
 
 import os
@@ -24,7 +23,6 @@ import types
 import numpy
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_SRC = "/root/reference/src"
 
 
 def _install_stubs():
@@ -54,10 +52,10 @@ def _install_stubs():
     mod("distributed", Client=_Unavailable)
 
 
-def import_reference():
+def import_reference(ref_src):
     _install_stubs()
-    if REF_SRC not in sys.path:
-        sys.path.insert(0, REF_SRC)
+    if ref_src not in sys.path:
+        sys.path.insert(0, ref_src)
     # pylint: disable=import-outside-toplevel
     from ska_sdp_exec_swiftly import api, api_helper
     from ska_sdp_exec_swiftly.fourier_transform import core, fourier_algorithm
@@ -218,12 +216,88 @@ def golden_windows(core_mod):
     print("ref_windows.npz")
 
 
-def main():
-    api, api_helper, core_mod, _ = import_reference()
-    golden_1d(core_mod)
-    golden_2d(api, api_helper, core_mod)
-    golden_windows(core_mod)
+def golden_dropin(api, api_helper, core_mod, fourier_algorithm):
+    """What tests/test_emu_reference_dropin.py compares against.
+
+    * A forward + backward pass through the reference's task bodies at SMALL_PARAMS, facets
+      from ``default_rng(77)``, subgrid 7 of the cover: the subgrid, and the backward facets
+      at DROPIN_SAMPLES seeded pixels together with each facet's largest magnitude.
+    * The direct-DFT expectations of the reference's 2-D unit tests at TEST_PARAMS: the point
+      source facets (dense; they compress to almost nothing) and the subgrids at
+      DROPIN_SAMPLES seeded pixels.
+    """
+    p = SMALL_PARAMS
+    core = core_mod.SwiftlyCore(p["W"], p["N"], p["xM_size"], p["yN_size"])
+    yB, xA = p["yB_size"], p["xA_size"]
+    facet_cfgs = api_helper.make_full_cover_config(p["N"], yB, api.FacetConfig)
+    sg_cfgs = api_helper.make_full_cover_config(p["N"], xA, api.SubgridConfig)
+    rng = numpy.random.default_rng(77)
+    facets = [rand_c(rng, yB, yB) for _ in facet_cfgs]
+    BF_F = [core.prepare_facet(f, fc.off0, axis=0) for f, fc in zip(facets, facet_cfgs)]
+    sg = sg_cfgs[7]
+    NMBF_BF = [api_helper.extract_column(core, bf, sg.off0, fc.off1)
+               for bf, fc in zip(BF_F, facet_cfgs)]
+    contribs = [core.extract_from_facet(nb, sg.off1, axis=1) for nb in NMBF_BF]
+    subgrid = api_helper.sum_and_finish_subgrid(core, contribs, facet_cfgs, sg)
+    pieces = api_helper.prepare_and_split_subgrid(core, subgrid, [sg.off0, sg.off1], facet_cfgs)
+    cols = [api_helper.accumulate_column(core, pc, None, sg.off1) for pc in pieces]
+    accs = [api_helper.accumulate_facet(core, c, None, fc, sg.off0)
+            for c, fc in zip(cols, facet_cfgs)]
+    back = numpy.array([api_helper.finish_facet(core, a, fc) for a, fc in zip(accs, facet_cfgs)])
+    pick = numpy.random.default_rng(78)
+    back_idx = numpy.sort(pick.choice(yB * yB, DROPIN_SAMPLES, replace=False))
+    out = {"tb_subgrid": subgrid, "tb_back_idx": back_idx,
+           "tb_back": back.reshape(len(back), -1)[:, back_idx],
+           "tb_back_scale": numpy.abs(back).max(axis=(1, 2))}
+
+    t = TEST_PARAMS
+    N, yB, xA = t["N"], t["yB_size"], t["xA_size"]
+    tcore = core_mod.SwiftlyCore(t["W"], N, t["xM_size"], t["yN_size"])
+    Nx, Ny = tcore.subgrid_off_step, tcore.facet_off_step
+    sg_idx = numpy.sort(pick.choice(xA * xA, DROPIN_SAMPLES, replace=False))
+    out["dft_sg_idx"] = sg_idx
+    # facet -> subgrid: point sources in facets, direct DFT of the subgrids
+    f2s_sources, s2f_sources = dropin_sources()
+    offs_f = [[0, 0], [Ny, Ny], [-Ny, Ny], [0, -Ny]]
+    offs_s = [[0, 0], [0, Nx], [Nx, 0], [-Nx, -Nx]]
+    out["f2s_facets"] = numpy.array([
+        fourier_algorithm.make_facet_from_sources(src, N, yB, fo)
+        for src in f2s_sources for fo in offs_f])
+    out["f2s_subgrids"] = numpy.array([
+        fourier_algorithm.make_subgrid_from_sources(src, N, xA, so).reshape(-1)[sg_idx]
+        for src in f2s_sources for so in offs_s])
+    # subgrid -> facet: DFT subgrids in, point sources in the facets expected
+    out["s2f_subgrids"] = numpy.array([
+        fourier_algorithm.make_subgrid_from_sources(src, N, xA, so).reshape(-1)[sg_idx]
+        for src in s2f_sources for so in offs_s])
+    out["s2f_facets"] = numpy.array([
+        fourier_algorithm.make_facet_from_sources(src, N, yB, fo)
+        for src in s2f_sources for fo in offs_f])
+    numpy.savez_compressed(os.path.join(HERE, "ref_dropin.npz"), **out)
+    print("ref_dropin.npz")
+
+
+DROPIN_SAMPLES = 2048
+
+
+def dropin_sources():
+    """Point sources (intensity, position 0, position 1) of the reference's 2-D unit tests:
+    facet -> subgrid, subgrid -> facet."""
+    return ([[(1, 1, 2)], [(1 / 8, 20, 4), (2 / 8, 2, 5), (3 / 8, -5, -4)]],
+            [[(1, 0, 0)], [(1, 20, 4)], [(3, -5, 4)]])
+
+
+def main(ref_src, names=()):
+    api, api_helper, core_mod, fourier_algorithm = import_reference(ref_src)
+    makers = {
+        "1d": lambda: golden_1d(core_mod),
+        "2d": lambda: golden_2d(api, api_helper, core_mod),
+        "windows": lambda: golden_windows(core_mod),
+        "dropin": lambda: golden_dropin(api, api_helper, core_mod, fourier_algorithm),
+    }
+    for name in names or makers:
+        makers[name]()
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1], sys.argv[2:])
